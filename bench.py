@@ -8,9 +8,13 @@ fp32 storage with TF32 tensor-core multiplies (the reference model is fp32; ``--
 Topology: every listed worker trains (/root/reference/distributed_mnist.py:27-29,120-122): N GPUs = N workers,
 ps shard s shares worker s's GPU; ``--ps-only-task 1`` gives the ps its own GPU (1 ps + (N-1) workers).
 
-* ``value``: whole-job samples/sec.  A repetition = EXACTLY K steps (one CUDA-graph replay chain) between CUDA events on
-  every rank's stream, after a barrier + synchronize and two untimed alignment steps; MAX over ranks per repetition;
-  repetitions continue until >= 100 ms of timed region were collected; the MEDIAN repetition is reported (``reps``).
+* ``value``: whole-job samples/sec.  The timed region is EXACTLY K steps, run as ``reps`` equal repetitions (up to 10, each
+  at least 100 steps when K allows; one CUDA-graph replay chain each) between CUDA events on every rank's stream, after a
+  barrier + synchronize and two untimed alignment steps; MAX over ranks per repetition; the MEDIAN repetition is reported.
+  The step count does not depend on timing, so a run with the same arguments computes the same steps.
+* ``--dump-outputs DIR``: after the timed steps, what they computed -- the loss of the last step, the parameters and optimizer
+  slots a caller would read back (``PSTrainEngine.state_dict``) -- as ``DIR/<name>.npy`` (float32 / float64, <= 64 MB in all),
+  so that two builds can be compared output for output.
 * inputs: a 55 000 x 784 fp32 synthetic MNIST-shaped training set resident in each worker's HBM
   (172 MB > the 126 MB L2), batches walked in order; the step kernel's TMA reads them in place.
 * ``e2e``: the same metric through the public API with, every step, the host->device copy of that step's batch from pinned host
@@ -63,7 +67,7 @@ def parse_args():
     ap.add_argument("--precision", default="tf32", choices=["tf32", "bf16"],
                     help="tf32: fp32 storage, TF32 MMAs, one-kernel worker step (reference precision); bf16: config 3")
     ap.add_argument("--step-ctas", type=int, default=0, help="tf32: CTAs of the step kernel (0: widest even split of the features)")
-    ap.add_argument("--min-ms", type=float, default=100.0, help="collect at least this much timed region (repetitions of K steps)")
+    ap.add_argument("--min-ms", type=float, default=100.0, help="e2e arms: collect at least this much timed region (repetitions of K steps)")
     ap.add_argument("--max-reps", type=int, default=400)
     ap.add_argument("--baseline", type=int, default=1, help="1: also time the torch+NCCL+cuBLAS arm in this invocation -> vs_baseline")
     ap.add_argument("--e2e-native-loop", type=int, default=1,
@@ -90,6 +94,8 @@ def parse_args():
     ap.add_argument("--placement", default="greedy", choices=["round_robin", "greedy"],
                     help="ResNet-18 variables -> ps shards: replica_device_setter's round robin, or its GreedyLoadBalancingStrategy "
                          "by bytes (creation order, least-loaded shard)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed (last loss, parameters, optimizer slots) as DIR/<name>.npy")
     ap.add_argument("--model", default="mnist_mlp", choices=["mnist_mlp", "resnet18"],
                     help="resnet18: BASELINE.json config 5 (conv model under the same ps API; bandwidth-relevant: 44.7 MB per push)")
     ap.add_argument("--nvls", default="auto", choices=["off", "on", "auto"],
@@ -237,6 +243,32 @@ class ClockSampler:
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": float(inside[0][2]), "reasons": reasons,
                 "samples": len(inside), "source": "nvidia-smi", "power_w_max": max(float(f[3]) for f in inside if f[3].replace(".", "").isdigit())
                 if any(f[3].replace(".", "").isdigit() for f in inside) else None}
+
+
+def repetition_plan(K: int):
+    """(repetitions, steps per repetition) of a timed region of exactly K steps: the most repetitions (<= 10) of equal length
+    that keep each at >= 100 steps, so that a repetition is long against the launch of its first graph."""
+    reps = max([r for r in range(1, 11) if K % r == 0 and K // r >= 100] or [1])
+    return reps, K // reps
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays) -> None:
+    """``arrays``: name -> array.  Written as ``out_dir/<name>.npy`` in float32 (float64 stays float64); when they exceed
+    DUMP_BYTES in all, every array is cut to its share by a fixed, seeded sample of its elements (same positions every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {n: np.asarray(a, dtype=np.float64 if np.asarray(a).dtype == np.float64 else np.float32) for n, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, int(a.size * DUMP_BYTES // total))
+            if keep < a.size:
+                idx = np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))
+                a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name.replace("/", "_") + ".npy"), a)
 
 
 def reference_arm(args):
@@ -694,8 +726,9 @@ def main():
         return [float(v) for v in t]
 
     K, W = args.steps, max(args.warmup, 3)
+    n_reps, k_rep = repetition_plan(K)
     use_graph = not args.no_graph
-    unroll = args.unroll or next(u for u in (50, 40, 32, 25, 20, 16, 10, 8, 5, 4, 2, 1) if K % u == 0)
+    unroll = args.unroll or next(u for u in (50, 40, 32, 25, 20, 16, 10, 8, 5, 4, 2, 1) if k_rep % u == 0)
     # ---- warm-up (eager: first-launch setup) + graph capture + graph warm-up ---------------------------------
     eng.enqueue_local_steps(W, "dataset")
     barrier()
@@ -720,18 +753,18 @@ def main():
 
     def k_steps():
         if use_graph:
-            eng.replay_graphs(K // unroll)
-            if K % unroll:
-                eng.enqueue_local_steps(K % unroll, "dataset")
+            eng.replay_graphs(k_rep // unroll)
+            if k_rep % unroll:
+                eng.enqueue_local_steps(k_rep % unroll, "dataset")
         else:
-            eng.enqueue_local_steps(K, "dataset")
+            eng.enqueue_local_steps(k_rep, "dataset")
 
     def measure(body):
-        """Repetitions of EXACTLY K steps: barrier + synchronize, two untimed alignment steps (the sync protocol itself lines
-        the ranks up, so the start skew of the barrier release is not part of the measurement), CUDA events on every local
-        stream around the K steps, MAX over ranks; until >= --min-ms of timed region (at least 3, at most --max-reps)."""
-        times, total = [], 0.0
-        while len(times) < 3 or (total < args.min_ms and len(times) < args.max_reps):
+        """``n_reps`` repetitions of ``k_rep`` steps (K in all): barrier + synchronize, two untimed alignment steps (the sync
+        protocol itself lines the ranks up, so the start skew of the barrier release is not part of the measurement), CUDA
+        events on every local stream around the repetition's steps, MAX over ranks."""
+        times = []
+        for _ in range(n_reps):
             barrier()
             align_steps()
             evs = []
@@ -746,7 +779,6 @@ def main():
                 e1.record(rk.stream)
             eng.synchronize()
             times.append(allmax([max(e0.elapsed_time(e1) for e0, e1, _ in evs)])[0])
-            total += times[-1]
         return times
 
     # ---- timed region ---------------------------------------------------------------------------------------
@@ -761,13 +793,13 @@ def main():
     t1 = time.time()
     clocks = sampler.stop(t0, t1)
     reps = len(times)
-    # kernels launched by the timed K-step regions only (the alignment steps are untimed and not counted)
-    per_rep = (cuda_lib.launch_count() - launches0) // reps
+    # kernels launched by the K timed steps only (the alignment steps are untimed and not counted)
+    launched = cuda_lib.launch_count() - launches0
     per_align = 2 * sum((eng.launches_per_worker_step("dataset") if r in eng.worker_ranks else 0) +
                         ((1 if cfg.sync else num_workers) if r in eng.ps_ranks else 0) for r in eng.ranks)
-    launches = per_rep - per_align
+    launches = launched - reps * per_align
     eng.check_errors()
-    ms = statistics.median(times)
+    ms = statistics.median(times) * n_reps           # a K-step region at the median repetition's rate
     st = torch.tensor([float(launches)], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(st, op=dist.ReduceOp.SUM)
@@ -777,6 +809,10 @@ def main():
     loss = allmax([loss if loss is not None else -1e30])[0]
     gstep = eng.read_ctl(0, "global_step") if 0 in eng.ranks else None
     stale = eng.staleness() if (args.mode == "async" and 0 in eng.ranks) else None
+    if args.dump_outputs and rank == 0:
+        sd = eng.state_dict()
+        dump_outputs(args.dump_outputs, dict({"loss": [loss]}, **{k: v.double().numpy() if k == "global_step" else v.float().numpy()
+                                                                   for k, v in sd.items()}))
 
     # ---- ps traffic implied by the measured step time (BASELINE metric: push/pull GB/s vs 900 GB/s/dir) -----------
     # true-shape bytes: gradients travel as fp32, parameters as fp32 (tf32 engines) / bf16 replicas; every worker moves both every step.
@@ -801,7 +837,7 @@ def main():
             "dtype": args.precision,
             "data": "synthetic MNIST-shaped 28x28 (55000x784 fp32 in HBM), random-init weights",
             "impl": "ours", "reps": reps, "timed_ms_total": sum(times),
-            "ms_per_step_min_max": [min(times) / K, max(times) / K],
+            "ms_per_step_min_max": [min(times) / k_rep, max(times) / k_rep],
             "config": {"model": "MNIST MLP 784-%d-10, clipped batch-sum xent" % spec.hidden,
                        "global_batch": num_workers * spec.batch, "per_worker_batch": spec.batch,
                        "parallelism": ("ps1+worker1 colocated on one GPU" if N == 1 else "ps%d+worker%d %s%s" % (
@@ -812,7 +848,8 @@ def main():
                                      else "bf16 operands, fp32 accumulate"),
                        "worker_step": ("one kernel (csrc/mlp_step.cu)" if args.precision == "tf32" else "stage + GEMM + head + GEMM"),
                        "l2": "inputs larger than L2: 172 MB fp32 train split cycled in HBM",
-                       "timing": "median of %d repetitions of exactly %d steps, each after barrier + 2 untimed alignment steps" % (reps, K),
+                       "timing": "median of %d repetitions of exactly %d steps (%d timed steps), each after barrier + 2 untimed "
+                                 "alignment steps" % (reps, k_rep, K),
                        "cuda_graph_unroll": unroll if use_graph else 0,
                        "pull": ("nvls multimem.st publish into fp32/bf16 replicas" if nvls_on and mc_on
                                 else "publish-replicas" if (args.publish or nvls_on) else "peer-pull by TMA inside the step / GEMM kernel"),

@@ -14,9 +14,10 @@
 //            pre-activation [128, H] of the slice in TMEM; it is written to a scratch buffer in L2.
 //   phase 2  (after a device-scope counter says all G partials landed) CTA c finalises batch rows [c*R, c*R + R):
 //            h = relu(sum of partials + b1), logits, softmax, loss, dlogits, dh rows (-> scratch), and its partial
-//            sums of dW2 / db2 / db1, which go into the gradient slot with fp32 atomics (the ps clears those ranges
-//            after reading them).
-//   phase 3  (after a second counter) TMA-loads all of dh; dW1^T[H, slice] = dh^T . x_slice with the SAME slice of the
+//            sums of dW2 / db2 / db1 (-> scratch).
+//   phase 3  (after a second counter) CTA c sums its share of the G head partials in CTA order and stores it into the
+//            gradient slot (a fixed order of additions: the step is bitwise reproducible, unlike fp32 atomics);
+//            TMA-loads all of dh; dW1^T[H, slice] = dh^T . x_slice with the SAME slice of the
 //            batch, re-fetched from L2 into the same shared-memory buffer while phase 2 runs (tcgen05 wants 32-bit
 //            MN-major operands in the SWIZZLE_128B_BASE32B arrangement, the K-major A of phase 1 in SWIZZLE_128B: same
 //            bytes, different swizzle, so TMA writes them twice); the epilogue stores the slice's rows of dW1 from TMEM
@@ -45,6 +46,8 @@ namespace dtf {
 
 static constexpr int kStepThreads = 256;
 static constexpr int kXChunkBytes = 128 * 128;     // one 32-feature-wide chunk of the batch tile: 128 rows x 128 bytes
+// one CTA's partial sums of the head gradients: dW2 [128][16], then db2 [16], then db1 [128]
+static constexpr int kHeadPart = 128 * 16 + 16 + 128;
 
 struct MlpStepParams {
   int B, D, H, C;              // batch <= 128, input features, hidden <= 128, classes <= 16
@@ -71,6 +74,7 @@ struct MlpStepParams {
   long long lddh;
   unsigned int* flags;         // [8]: {partials written, dh rows written, CTAs finished (all monotonic: G per launch), launch
                                //       epoch} for training launches, the same four again for forward-only launches
+  float* head_part;            // [G][kHeadPart] per-CTA partial sums of dW2 / db2 / db1
   // ---- gradient slots
   float* gw1;                  // [D, ldgw1]
   long long ldgw1;
@@ -580,32 +584,31 @@ __global__ void __launch_bounds__(kStepThreads, 1) mlp_step_kernel(DTF_STEP_MAPS
         s_dh[rg * 128 + j] = db1;                                // combine the two row groups below
       }
       STAMP(17);
-      // dW2[j][4cq .. 4cq+3] += sum_r h[r][j] * dl[r][4cq .. 4cq+3]: one scalar + one 16-byte load per 4 FMAs
+      // this CTA's partials of dW2[j][4cq .. 4cq+3] = sum_r h[r][j] * dl[r][4cq .. 4cq+3]: one scalar + one 16-byte load
+      // per 4 FMAs; db2 and db1 behind them (phase 3 adds the G partials up)
+      float* part = p.head_part + (long long)cta * kHeadPart;
       for (int it = tid; it < 128 * 4; it += kStepThreads) {
         const int j = it >> 2, cq = it & 3;
+        float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
         if (j < p.H && 4 * cq < p.C) {
-          float a[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
           for (int r = 0; r < 16; ++r) {                         // row slots beyond nrows hold zeros in s_h and s_dl
             const float hv = s_h[r * HP + j];
             const float4 d4 = *reinterpret_cast<const float4*>(s_dl + r * 16 + 4 * cq);
-            a[0] = fmaf(hv, d4.x, a[0]); a[1] = fmaf(hv, d4.y, a[1]); a[2] = fmaf(hv, d4.z, a[2]); a[3] = fmaf(hv, d4.w, a[3]);
+            a.x = fmaf(hv, d4.x, a.x); a.y = fmaf(hv, d4.y, a.y); a.z = fmaf(hv, d4.z, a.z); a.w = fmaf(hv, d4.w, a.w);
           }
-          float* gw = p.gw2 + (long long)j * p.ldgw2 + 4 * cq;
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            if (4 * cq + k < p.C) atomicAdd(gw + k, a[k]);
         }
+        reinterpret_cast<float4*>(part)[it] = a;
       }
-      if (tid < p.C) {
+      if (tid < 16) {
         float a = 0.f;
 #pragma unroll
         for (int r = 0; r < 16; ++r) a += s_dl[r * 16 + tid];
-        atomicAdd(p.gb2 + tid, a);
+        part[128 * 16 + tid] = a;
       }
       __syncthreads();
       STAMP(18);
-      if (tid < p.H) atomicAdd(p.gb1 + tid, s_dh[tid] + s_dh[128 + tid]);
+      if (tid < 128) part[128 * 16 + 16 + tid] = s_dh[tid] + s_dh[128 + tid];
 #ifndef DTF_HOST_EMU
       if (fused && p.clustered) {
         STAMP(19);
@@ -653,10 +656,36 @@ __global__ void __launch_bounds__(kStepThreads, 1) mlp_step_kernel(DTF_STEP_MAPS
       }
       umma_commit(bar_m2);
     }
-    mbar_wait(bar_m2, 0);
-    tc_fence_after();
 #else
     if (fused) { /* emulated blocks run one after another: the fused mode is hardware-only */ }
+#endif
+    // while the MMAs run: the head gradients of this CTA's share of [0, kHeadPart), the G partials added in CTA order.
+    // Thread 0 acquired the phase-2 counter above (clustered: the cluster barrier did), so every partial is in L2
+    __syncthreads();
+    {
+      const int share = (kHeadPart + p.G - 1) / p.G;
+      const int e_hi = min(kHeadPart, (cta + 1) * share);
+      for (int e = cta * share + tid; e < e_hi; e += kStepThreads) {
+        float* dst;
+        if (e < 128 * 16) dst = (e / 16 < p.H && e % 16 < p.C) ? p.gw2 + (long long)(e / 16) * p.ldgw2 + e % 16 : nullptr;
+        else if (e < 128 * 16 + 16) dst = (e - 128 * 16 < p.C) ? p.gb2 + (e - 128 * 16) : nullptr;
+        else dst = (e - 128 * 16 - 16 < p.H) ? p.gb1 + (e - 128 * 16 - 16) : nullptr;
+        if (dst == nullptr) continue;
+        const float* src = p.head_part + e;
+        float a = 0.f;
+        for (int c0 = 0; c0 < p.G; c0 += 8) {
+          float t[8];
+#pragma unroll
+          for (int u = 0; u < 8; ++u) t[u] = (c0 + u < p.G) ? __ldcg(src + (long long)(c0 + u) * kHeadPart) : 0.f;
+#pragma unroll
+          for (int u = 0; u < 8; ++u) a += t[u];
+        }
+        *dst = a;
+      }
+    }
+#ifndef DTF_HOST_EMU
+    mbar_wait(bar_m2, 0);
+    tc_fence_after();
 #endif
     STAMP(7);
     // epilogue 2: TMEM (lane = hidden unit j, column = feature i of the slice) -> gw1[d0 + i][j]: a warp stores 32
@@ -725,7 +754,7 @@ __global__ void __launch_bounds__(kStepThreads, 1) mlp_step_kernel(DTF_STEP_MAPS
     STAMP(8);
     if (tid == 0) {
       // CTA 0 stamps the push FIRST; then ONE fence by one thread per CTA after the CTA barrier (release is cumulative: it
-      // covers the bulk store waited for above, the head's atomics and the stamp), then a RELAXED arrival.  The ps acts on
+      // covers the bulk store waited for above, the head's stores and the stamp), then a RELAXED arrival.  The ps acts on
       // the push only once all G arrivals are in, CTA 0's included, so the stamp is visible by then.  When the ps shares this
       // GPU AND this stream (colocated), its kernel starts after this one has completed: no fence at all.
       if (cta == 0)
@@ -806,6 +835,7 @@ struct DtfMlpStepArgs {
   int no_cluster;              // 1: plain grid + L2 counters even when the CTAs would fit one cluster
   int dbg;
   unsigned long long* ring; int ring_cap;      // optional worker trace ring: (ring_cap + 1) rows of 8 u64
+  float* head_part;            // [G][dtf_mlp_step_head_part_floats()] scratch (training launches)
 };
 
 // Slices: at least ceil(B / 16) CTAs (phase 2 finalises <= 16 batch rows per CTA), at most 16; among those the widest
@@ -861,6 +891,8 @@ int dtf_mlp_step(const DtfMlpStepArgs* a, cudaStream_t s) {
   p.w1 = a->w1; p.ldw1 = a->ldw1; p.b1 = a->b1; p.w2 = a->w2; p.ldw2 = a->ldw2; p.b2 = a->b2;
   p.hpart = a->hpart; p.dh = a->dh; p.lddh = a->lddh; p.flags = a->flags;
   p.gw1 = a->gw1; p.ldgw1 = a->ldgw1; p.gb1 = a->gb1; p.gw2 = a->gw2; p.ldgw2 = a->ldgw2; p.gb2 = a->gb2;
+  p.head_part = a->head_part;
+  if (!a->forward_only && a->head_part == nullptr) return -3;
   p.clip_min = a->clip_min; p.loss_out = a->loss_out; p.logits_out = a->logits_out;
   p.step_counter = a->step_counter; p.forward_only = a->forward_only;
   if (a->num_tokens > 4 || a->num_signals > 4) return -2;
@@ -949,5 +981,6 @@ int dtf_mlp_step(const DtfMlpStepArgs* a, cudaStream_t s) {
 }
 
 int dtf_sizeof_mlp_step_args() { return (int)sizeof(DtfMlpStepArgs); }
+int dtf_mlp_step_head_part_floats() { return kHeadPart; }
 
 }  // extern "C"

@@ -86,7 +86,8 @@ class MlpStepArgs(Structure):
                 ("token_base", c_ulonglong * 4), ("stamp_step", c_int), ("consumed", c_void_p * 4),
                 ("num_signals", c_int), ("arrivals", c_void_p * 4), ("stamp_dst", c_void_p * 4), ("stamp_src", c_void_p * 4),
                 ("sys_scope", c_int), ("timeout_ns", c_ulonglong), ("err", c_void_p), ("trace", c_void_p),
-                ("no_cluster", c_int), ("dbg", c_int), ("ring", c_void_p), ("ring_cap", c_int)]
+                ("no_cluster", c_int), ("dbg", c_int), ("ring", c_void_p), ("ring_cap", c_int),
+                ("head_part", c_void_p)]
 
 
 class StepOp(Structure):
@@ -265,6 +266,7 @@ def _declare(lib) -> None:
         lib.dtf_mlp_step_scratch_floats.argtypes = [c_int, c_int, c_int]
         lib.dtf_mlp_step_scratch_floats.restype = c_longlong
         lib.dtf_sizeof_mlp_step_args.restype = c_int
+        lib.dtf_mlp_step_head_part_floats.restype = c_int
         assert lib.dtf_sizeof_mlp_step_args() == ctypes.sizeof(MlpStepArgs), "MlpStepArgs layout mismatch"
     lib.dtf_run_ops.argtypes = [c_void_p, c_int, c_int, c_void_p, c_void_p]
     lib.dtf_run_ops.restype = c_int

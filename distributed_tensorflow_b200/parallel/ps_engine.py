@@ -299,8 +299,10 @@ class PSTrainEngine:
                          ("h_w%d" % w, 128 * ldh * 2), ("dh_w%d" % w, 128 * ldh * 2), ("hacc_w%d" % w, 128 * ldh * 4),
                          ("misc_w%d" % w, 4096 + cfg.loss_hist * 4)]
                 if self.tf32:
-                    # scratch of the one-kernel step: partial pre-activations + dh (L2 resident), 8 sync counters, phase stamps
-                    nfl = self.step_ctas * 128 * (round_up(spec.hidden, 16) + 4) + 128 * 128 + 64
+                    # scratch of the one-kernel step: partial pre-activations + dh + partial head gradients (L2 resident),
+                    # 8 sync counters, phase stamps
+                    nfl = (self.step_ctas * 128 * (round_up(spec.hidden, 16) + 4) + 128 * 128 + 64
+                           + self.step_ctas * int(self.lib.dtf_mlp_step_head_part_floats()))
                     names += [("stepscr_w%d" % w, nfl * 4), ("stepflags_w%d" % w, 256), ("steptrace_w%d" % w, 16 * 32 * 8),
                               ("stepring_w%d" % w, (cfg.worker_trace_cap + 1) * 64)]
                 for s in range(cfg.num_ps):
@@ -700,6 +702,7 @@ class PSTrainEngine:
         a.w1, a.ldw1, a.b1 = k["w1"], k["ldw1"], k["b1"]
         a.w2, a.ldw2, a.b2 = k["w2"], k["ldw2"], k["b2"]
         a.hpart, a.dh, a.lddh = k["scr"], k["scr"] + self.step_ctas * 128 * (round_up(spec.hidden, 16) + 4) * 4, 128
+        a.head_part = a.dh + (128 * 128 + 64) * 4
         a.flags = k["flags"]
         a.gw1, a.ldgw1, a.gb1 = k["gw1"], lay["hid_w"].pitch, k["gb1"]
         a.gw2, a.ldgw2, a.gb2 = k["gw2"], lay["sm_w"].pitch, k["gb2"]

@@ -66,9 +66,11 @@ def test_step_kernel_matches_float64_model(B, D, H, C, nbatches, wide, mask):
     n1 = (H + 15) // 16 * 16
     hpart = torch.zeros(G * 128 * (n1 + 4), device=dev)
     dh = torch.zeros(128, 128, device=dev)
+    head_part = torch.zeros(G * lib.dtf_mlp_step_head_part_floats(), device=dev)
     flags = torch.zeros(8, dtype=torch.int32, device=dev)
-    gw1, gb1 = torch.full((D, ldw1), 7.0, device=dev), torch.zeros(H, device=dev)
-    gw2, gb2 = torch.zeros(H, ldw2, device=dev), torch.zeros(C, device=dev)
+    # every gradient is STORED: stale content of the slot must be overwritten
+    gw1, gb1 = torch.full((D, ldw1), 7.0, device=dev), torch.full((H,), 7.0, device=dev)
+    gw2, gb2 = torch.full((H, ldw2), 7.0, device=dev), torch.full((C,), 7.0, device=dev)
     loss, logits = torch.zeros(16, device=dev), torch.zeros(B, C, device=dev)
     step0 = 1 if nbatches else 0
     stepctr = torch.tensor([step0], dtype=torch.int64, device=dev)
@@ -87,6 +89,7 @@ def test_step_kernel_matches_float64_model(B, D, H, C, nbatches, wide, mask):
     a.w1, a.ldw1, a.b1, a.w2, a.ldw2, a.b2 = p(w1), ldw1, p(b1), p(w2), ldw2, p(b2)
     a.hpart, a.dh, a.lddh, a.flags = p(hpart), p(dh), 128, p(flags)
     a.gw1, a.ldgw1, a.gb1, a.gw2, a.ldgw2, a.gb2 = p(gw1), ldw1, p(gb1), p(gw2), ldw2, p(gb2)
+    a.head_part = p(head_part)
     a.clip_min, a.loss_out, a.logits_out, a.step_counter = 1e-10, p(loss), p(logits), p(stepctr)
     a.num_tokens, a.token[0] = 1, p(token)
     a.num_signals, a.arrivals[0], a.stamp_dst[0], a.stamp_src[0] = 1, p(arrivals), p(arrivals) + 8, p(token)
@@ -132,6 +135,7 @@ def test_step_kernel_two_consecutive_steps_and_forward_only():
     b1, b2 = torch.zeros(H, device=dev), torch.zeros(C, device=dev)
     G = lib.dtf_mlp_step_slices(D, B, None)
     hpart, dh = torch.zeros(G * 128 * 116, device=dev), torch.zeros(128, 128, device=dev)
+    head_part = torch.zeros(G * lib.dtf_mlp_step_head_part_floats(), device=dev)
     flags = torch.zeros(8, dtype=torch.int32, device=dev)
     gw1, gb1, gw2, gb2 = (torch.zeros(s, device=dev) for s in ((D, 104), (H,), (H, 16), (C,)))
     loss, logits = torch.zeros(16, device=dev), torch.zeros(B, C, device=dev)
@@ -147,13 +151,14 @@ def test_step_kernel_two_consecutive_steps_and_forward_only():
     a.w1, a.ldw1, a.b1, a.w2, a.ldw2, a.b2 = p(w1), 104, p(b1), p(w2), 16, p(b2)
     a.hpart, a.dh, a.lddh, a.flags = p(hpart), p(dh), 128, p(flags)
     a.gw1, a.ldgw1, a.gb1, a.gw2, a.ldgw2, a.gb2 = p(gw1), 104, p(gb1), p(gw2), 16, p(gb2)
+    a.head_part = p(head_part)
     a.clip_min, a.loss_out, a.logits_out, a.step_counter = 1e-10, p(loss), p(logits), p(stepctr)
     a.num_tokens, a.token[0] = 1, p(token)
     a.num_signals, a.arrivals[0], a.stamp_dst[0], a.stamp_src[0] = 1, p(arrivals), p(arrivals) + 8, p(token)
     a.sys_scope, a.timeout_ns, a.err = 0, 2 * 10**9, p(err)
     st = torch.cuda.current_stream().cuda_stream
     for t in range(2):
-        gw2.zero_(); gb2.zero_(); gb1.zero_()                       # what the ps does after reading the accumulated ranges
+        gw2.fill_(7.0); gb2.fill_(7.0); gb1.fill_(7.0)              # the step overwrites what the previous one left
         assert lib.dtf_mlp_step(ctypes.byref(a), st) == 0
         torch.cuda.synchronize()
         ref_loss, _, ref = _reference(xs_h[t * B:(t + 1) * B], ys_h[t * B:(t + 1) * B], w1_h[:, :H], b1.cpu(), w2_h[:, :C], b2.cpu())

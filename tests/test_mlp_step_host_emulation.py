@@ -1,7 +1,7 @@
 """The one-kernel worker step (csrc/mlp_step.cu) under the host emulation: same source, the TMA / tcgen05 parts replaced by
 scalar loops, the three phases launched one after another (emulated blocks run sequentially).  Checks everything around the
 tensor-core tiles -- slice / row ownership, the L2 exchange buffers, the fused head (softmax, clipped batch-SUM
-cross-entropy, dlogits, dh, dW2 / db2 / db1 partial sums with atomics), the dW1 store pattern, the device step counter,
+cross-entropy, dlogits, dh, dW2 / db2 / db1 partial sums added in CTA order), the dW1 store pattern, the device step counter,
 stamp + arrival -- against a float64 PyTorch model of /root/reference/distributed_mnist.py:109-113."""
 import ctypes
 import shutil
@@ -56,9 +56,11 @@ def test_step_kernel_matches_float64_model(emu, B, D, H, C, nbatches):
     n1 = (H + 15) // 16 * 16
     hpart = torch.zeros(G * 128 * (n1 + 4))
     dh = torch.zeros(128, 128)
+    head_part = torch.zeros(G * emu.dtf_mlp_step_head_part_floats())
     flags = torch.zeros(8, dtype=torch.int32)
-    gw1, gb1 = torch.full((D, ldw1), 7.0), torch.zeros(H)          # dW1 is STORED (stale content must be overwritten) ...
-    gw2, gb2 = torch.zeros(H, ldw2), torch.zeros(C)                # ... the head's sums are ACCUMULATED (the ps clears them)
+    # every gradient is STORED (stale content must be overwritten); the head's sums in a fixed order of the CTA partials
+    gw1, gb1 = torch.full((D, ldw1), 7.0), torch.full((H,), 7.0)
+    gw2, gb2 = torch.full((H, ldw2), 7.0), torch.full((C,), 7.0)
     loss = torch.zeros(16)
     logits = torch.zeros(B, C)
     stepctr = torch.tensor([1 if nbatches else 0], dtype=torch.int64)
@@ -73,6 +75,7 @@ def test_step_kernel_matches_float64_model(emu, B, D, H, C, nbatches):
     a.w1, a.ldw1, a.b1, a.w2, a.ldw2, a.b2 = _ptr(w1), ldw1, _ptr(b1), _ptr(w2), ldw2, _ptr(b2)
     a.hpart, a.dh, a.lddh, a.flags = _ptr(hpart), _ptr(dh), 128, _ptr(flags)
     a.gw1, a.ldgw1, a.gb1, a.gw2, a.ldgw2, a.gb2 = _ptr(gw1), ldw1, _ptr(gb1), _ptr(gw2), ldw2, _ptr(gb2)
+    a.head_part = _ptr(head_part)
     a.clip_min, a.loss_out, a.logits_out, a.step_counter = 1e-10, _ptr(loss), _ptr(logits), _ptr(stepctr)
     a.num_tokens, a.token[0] = 1, _ptr(token)
     a.num_signals, a.arrivals[0], a.stamp_dst[0], a.stamp_src[0] = 1, _ptr(arrivals), _ptr(arrivals) + 8, _ptr(token)

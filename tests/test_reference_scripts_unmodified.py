@@ -2,8 +2,9 @@
 (``distributed_tensorflow_b200/compat``): the strongest parity check available without TensorFlow -- every symbol,
 default, device string and hook protocol the scripts exercise has to behave (SURVEY section 2.2, A1-A23).
 
-Needs the read-only reference checkout at ``/root/reference`` (skipped elsewhere).  The scripts hard-code
-``localhost:2222-2224`` / explicit host flags, so these tests must not run concurrently with each other."""
+The scripts are not part of this repository: those tests need a checkout of the reference project, named by
+``DTF_REFERENCE_DIR``, and skip without one.  The scripts hard-code ``localhost:2222-2224`` / explicit host flags, so these
+tests must not run concurrently with each other."""
 import os
 import subprocess
 import sys
@@ -13,8 +14,8 @@ import pytest
 
 REF = os.environ.get("DTF_REFERENCE_DIR", "/root/reference")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "distributed_mnist.py")),
-                                reason="reference checkout not available")
+needs_reference = pytest.mark.skipif(not os.path.exists(os.path.join(REF, "distributed_mnist.py")),
+                                     reason="reference checkout not available")
 
 
 def _env(tmp_path):
@@ -65,11 +66,13 @@ def _golden(out):
         assert v in flat, out
 
 
+@needs_reference
 def test_reference_standalone_py(tmp_path):
     out = _run(tmp_path, "standalone.py", timeout=600)           # 10 000 tower steps on one fixed batch
     assert "affine_last/w" in out and "GPU" in out               # '2块GPU用时: ...s'
 
 
+@needs_reference
 def test_reference_example_in_graph_py(tmp_path):
     with _Tasks(tmp_path) as t:
         t.start("example_in_graph.py", "--job_name=ps", "--task_index=0")
@@ -79,6 +82,7 @@ def test_reference_example_in_graph_py(tmp_path):
     assert (tmp_path / "timeline_client.json").exists() and (tmp_path / "logs").exists()
 
 
+@needs_reference
 def test_reference_distributed_server_and_client_py(tmp_path):
     with _Tasks(tmp_path) as t:
         t.start("example_distributed_server.py", "--job_name=ps", "--task_index=0")
@@ -100,6 +104,7 @@ def test_reference_distributed_server_and_client_py(tmp_path):
             p.wait(timeout=10)
 
 
+@needs_reference
 @pytest.mark.parametrize("sync", [True, False])
 def test_reference_example_between_graph_py(tmp_path, sync):
     hosts = ["--ps_hosts=127.0.0.1:22251", "--worker_hosts=127.0.0.1:22252,127.0.0.1:22253"]
@@ -115,6 +120,7 @@ def test_reference_example_between_graph_py(tmp_path, sync):
     assert (tmp_path / "hdfs" / "test" / "ckpt" / "checkpoint").exists()      # hdfs:// checkpoint dir mapped to a local root
 
 
+@needs_reference
 @pytest.mark.skipif(os.environ.get("DTF_SLOW_TESTS", "0") != "1", reason="10 000 global steps (~2 min): DTF_SLOW_TESTS=1")
 def test_reference_distributed_mnist_then_predict_py(tmp_path):
     hosts = ["--ps_hosts=127.0.0.1:22221", "--worker_hosts=127.0.0.1:22222,127.0.0.1:22223"]
